@@ -138,6 +138,24 @@ def images_per_sec_from_forward(sec_per_sample_forward: float, steps: int = 30) 
     return 1.0 / (2 * steps * sec_per_sample_forward)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname: str, arrays: dict) -> None:
+    """Write each array as DIR/<name>.npy in float32, all of them together within DUMP_LIMIT_BYTES: an array that does not
+    fit its share is replaced by a fixed, seeded sample of its flattened elements (the same positions in every run with
+    the same arguments, so that two builds can be compared output for output)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    share = (DUMP_LIMIT_BYTES - 4096 * len(arrays)) // len(arrays) // 4  # elements per array (.npy headers allowed for)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > share:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(dirname, name + ".npy"), a.numpy())
+
+
 def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -343,8 +361,11 @@ def run_flux(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item()) * 1e-3
 
+    last = {}
+
     def step_resident():
-        finish(job(devin))
+        last["images"] = job(devin)
+        finish(last["images"])
 
     def step_e2e():
         lat = job(host)
@@ -363,6 +384,7 @@ def run_flux(args):
     if os.environ.get("B200_PROFILE_TIMED"):
         torch.cuda.profiler.stop()
     launches = ops.LAUNCHES - l0
+    timed_out = last["images"].clone() if args.dump_outputs else None  # the next calls reuse the pipeline's output buffers
     step_e2e()
     sec_e2e = timed(step_e2e, K)
     clk = clocks.stop()
@@ -413,6 +435,8 @@ def run_flux(args):
                 "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
                 "gpu_launches": launches, "clocks": clk, "roofline": roof, "kernel_families": fam, "cpu_baseline": None}
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"images": timed_out})
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
@@ -438,7 +462,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (the decoded images [B, H, W, 3]; "
+                         "under torchrun, the batch rank 0 computed itself) as DIR/images.npy, float32; above 64 MB a fixed, "
+                         "seeded sample of its elements.  B200 arm only")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the B200 arm: the reference arm times UNet forwards, not whole jobs")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -585,8 +615,11 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item()) * 1e-3
 
+    last = {}
+
     def step_resident():
-        finish(job(devin))
+        last["images"] = job(devin)
+        finish(last["images"])
 
     def step_e2e_pipeline():
         img = job(host)
@@ -613,6 +646,7 @@ def main():
     if os.environ.get("B200_PROFILE_TIMED"):
         torch.cuda.profiler.stop()
     launches = ops.LAUNCHES - l0
+    timed_out = last["images"].clone() if args.dump_outputs else None  # the next calls reuse the pipeline's output buffers
     step_e2e()  # untimed: graph capture / first-call setup of this leg
     l1 = ops.LAUNCHES
     sec_e2e = timed(step_e2e, K)
@@ -759,6 +793,8 @@ def main():
             "attention_vs_sdpa": attn_pair,
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"images": timed_out})
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()

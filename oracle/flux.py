@@ -183,17 +183,22 @@ def flux_forward(sd: SD, cfg: dict, x: torch.Tensor, timestep: torch.Tensor, con
     return unpatchify(out, C, Hh, Ww)
 
 
-def random_state_dict(cfg: dict, seed: int = 0, dtype=torch.float32) -> SD:
+def random_state_dict(cfg: dict, seed: int = 0, dtype=torch.float32, device=None) -> SD:
     """Deterministic synthetic weights with the reference's parameter names and shapes (same conventions as
     oracle.unet.random_state_dict).  Modulation weights are scaled down so (1 + scale) stays near 1 and gates near
     0.3: the residual stream keeps O(1) magnitude through all blocks."""
     g = torch.Generator().manual_seed(seed)
+    assert device in (None, "cpu", "meta"), device
+
+    def randn(*shape):  # device="meta": names and shapes only, nothing drawn or allocated
+        return torch.empty(*shape, device="meta") if device == "meta" else torch.randn(*shape, generator=g)
+
     sd: SD = {}
 
     def lin(p, cin, cout, bias=True, wscale=1.0, bmean=0.0):
-        sd[p + ".weight"] = (torch.randn(cout, cin, generator=g) * (wscale * cin ** -0.5)).to(dtype)
+        sd[p + ".weight"] = (randn(cout, cin) * (wscale * cin ** -0.5)).to(dtype)
         if bias:
-            sd[p + ".bias"] = (bmean + torch.randn(cout, generator=g) * 0.05).to(dtype)
+            sd[p + ".bias"] = (bmean + randn(cout) * 0.05).to(dtype)
 
     hs, H = cfg["hidden_size"], cfg["num_heads"]
     D = hs // H
@@ -205,8 +210,8 @@ def random_state_dict(cfg: dict, seed: int = 0, dtype=torch.float32) -> SD:
     lin("txt_in", cfg["context_in_dim"], hs)
 
     def qknorm(p):
-        sd[p + ".query_norm.scale"] = (1.0 + 0.1 * torch.randn(D, generator=g)).to(dtype)
-        sd[p + ".key_norm.scale"] = (1.0 + 0.1 * torch.randn(D, generator=g)).to(dtype)
+        sd[p + ".query_norm.scale"] = (1.0 + 0.1 * randn(D)).to(dtype)
+        sd[p + ".key_norm.scale"] = (1.0 + 0.1 * randn(D)).to(dtype)
 
     for i in range(cfg["depth"]):
         p = f"double_blocks.{i}"

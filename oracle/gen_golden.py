@@ -21,8 +21,7 @@ if ROOT not in sys.path:
 from oracle import configs as CF  # noqa: E402
 from oracle import ref_import  # noqa: E402
 from oracle import unet as OU  # noqa: E402
-
-GOLD = os.path.join(ROOT, "tests", "golden")
+from oracle.golden import GOLD, control_residuals, sample_index, seeded_inputs  # noqa: E402
 
 
 def sd_checksum(sd) -> float:
@@ -381,15 +380,13 @@ def gen_unet_control(name: str = "tiny_xl", hw: int = 16):
         m(x, t, context=ctx, y=y, transformer_options={})
     for h in hooks:
         h.remove()
-    g = torch.Generator().manual_seed(19)
-    ins = [torch.randn(s, generator=g) * 0.3 for s in shapes["input"]]
-    control = {"input": list(reversed(ins)),                                   # popped from the end: block 0 first
-               "middle": [torch.randn(shapes["middle"][0], generator=g) * 0.3],
-               "output": [None if i == 2 else torch.randn(s, generator=g) * 0.3 for i, s in enumerate(shapes["input"])]}
+    control_shapes = {"input": shapes["input"], "middle": shapes["middle"][:1]}
+    control = control_residuals(control_shapes, seed=19)
     with torch.no_grad():
         out = m(x, t, context=ctx, y=y, control={k: list(v) for k, v in control.items()}, transformer_options={})
-    torch.save(dict(config=name, weight_seed=1, weight_checksum=sd_checksum(sd), x=x, t=t, context=ctx, y=y, control=control, out=out),
-               os.path.join(GOLD, f"unet_{name}_control.pt"))
+    # the residuals are not stored: control_residuals() regenerates them from the seed and shapes
+    torch.save(dict(config=name, weight_seed=1, weight_checksum=sd_checksum(sd), x=x, t=t, context=ctx, y=y,
+                    control_seed=19, control_shapes=control_shapes, out=out), os.path.join(GOLD, f"unet_{name}_control.pt"))
     print("unet control", name, "out std", out.std().item())
 
 
@@ -433,10 +430,258 @@ def gen_flux(name: str = "tiny_flux", hw: int = 16, txt_len: int = 128, fname: s
     print("flux", name, "out std", out.std().item())
 
 
+def gen_unet_b1(name: str = "tiny_xl"):
+    """A second reference UNet forward at other weights / shape / timestep: batch 1, 8 x 8 latent, t = 400."""
+    from backend.nn.unet import IntegratedUNet2DConditionModel as RefUNet
+    cfg = CF.CONFIGS[name]
+    sd = OU.random_state_dict(cfg, seed=5)
+    m = RefUNet(**cfg).eval()
+    m.load_state_dict(sd, strict=True)
+    g = torch.Generator().manual_seed(6)
+    x = torch.randn(1, 4, 8, 8, generator=g)
+    ctx = torch.randn(1, 77, cfg["context_dim"], generator=g)
+    y = torch.randn(1, cfg["adm_in_channels"], generator=g)
+    t = torch.tensor([400.0])
+    with torch.no_grad():
+        out = m(x, t, context=ctx, y=y, transformer_options={})
+    torch.save(dict(config=name, weight_seed=5, weight_checksum=sd_checksum(sd), x=x, t=t, context=ctx, y=y, out=out),
+               os.path.join(GOLD, f"unet_{name}_b1.pt"))
+    print("unet b1", name, "out std", out.std().item())
+
+
+def gen_param_shapes():
+    """Parameter names and shapes of the reference's full-size SD1.5 / SDXL UNets and Flux.1-dev transformer (built on
+    the meta device), stored as gzipped JSON {model: {name: shape}}."""
+    import gzip
+    import json
+
+    from backend.nn.flux import IntegratedFluxTransformer2DModel
+    from backend.nn.unet import IntegratedUNet2DConditionModel as RefUNet
+    from oracle import flux as OF
+    out = {}
+    for key, ctor in (("sd15", lambda: RefUNet(**CF.CONFIGS["sd15"])), ("sdxl", lambda: RefUNet(**CF.CONFIGS["sdxl"])),
+                      ("flux_dev", lambda: IntegratedFluxTransformer2DModel(**OF.FLUX_DEV))):
+        with torch.device("meta"):
+            m = ctor()
+        out[key] = {k: list(p.shape) for k, p in m.named_parameters()}
+        print("param shapes", key, len(out[key]), sum(p.numel() for p in m.parameters()))
+    with gzip.GzipFile(os.path.join(GOLD, "param_shapes.json.gz"), "wb", mtime=0) as f:
+        f.write(json.dumps(out, separators=(",", ":"), sort_keys=True).encode())
+
+
+def _detach(obj):
+    """Tensors cloned, containers walked, anything else dropped (callables, model handles in transformer_options)."""
+    if torch.is_tensor(obj):
+        return obj.detach().clone()
+    if isinstance(obj, dict):
+        return {k: _detach(v) for k, v in obj.items() if torch.is_tensor(v) or isinstance(v, (dict, list, tuple, int, float, str, bool, type(None)))}
+    if isinstance(obj, (list, tuple)):
+        return type(obj)(_detach(v) for v in obj)
+    return obj
+
+
+def _record_wrapper_call(kmodel, x, sigma, uc, cc, cfg_scale):
+    """Run the reference's sampling_function_inner with a model_function_wrapper that records what it is handed and what
+    the reference's own apply_model returns for it."""
+    from backend.sampling.sampling_function import sampling_function_inner
+    calls = []
+
+    def rec(apply_model, args):
+        out = apply_model(args["input"], args["timestep"], **args["c"])
+        calls.append(dict(args=_detach(args), out=out.detach().clone(), timestep_from_sigma=kmodel.predictor.timestep(args["timestep"]).clone()))
+        return out
+
+    with torch.no_grad():
+        base = sampling_function_inner(kmodel, x, sigma, uc, cc, cfg_scale, {}, None)
+        got = sampling_function_inner(kmodel, x, sigma, uc, cc, cfg_scale, {"model_function_wrapper": rec}, None)
+    assert torch.equal(base, got) and len(calls) == 1, len(calls)
+    return dict(calls[0], prediction_type=kmodel.predictor.prediction_type)
+
+
+def gen_plugin_calls():
+    """What the reference hands the plug points, and what its own code returns for it:
+    - P1: the modules that import attention_function by value, and the attention_pytorch result on one input; the
+      signature (shapes, heads, layout arguments) of each distinct attention call made by the reference UNet (tiny_xl) and
+      Flux transformer (tiny) forwards of unet_tiny_xl.pt / flux_tiny.pt, with a sample of the reference's result on
+      seeded inputs of those shapes;
+    - P3: the model_function_wrapper call made by sampling_function_inner for a tiny_xl UNet (CFG 7) and a tiny Flux
+      transformer (CFG 1), with the result of the reference's apply_model for the same arguments."""
+    import backend.attention as ba
+    import backend.nn.chroma  # noqa: F401
+    import backend.nn.flux as bf
+    import backend.nn.unet as bu
+    import backend.nn.vae  # noqa: F401
+    from backend.modules.k_model import KModel
+    from backend.modules.k_prediction import Prediction, PredictionFlux
+    from backend.sampling.condition import compile_conditions
+    from oracle import flux as OF
+    out = {}
+    out["attention_importers"] = sorted(n for n, m in list(sys.modules.items())
+                                        if m is not None and n != "backend.attention" and getattr(m, "attention_function", None) is ba.attention_function)
+    out["single_head_importers"] = sorted(n for n, m in list(sys.modules.items()) if m is not None and n != "backend.attention"
+                                          and getattr(m, "attention_function_single_head_spatial", None) is ba.attention_function_single_head_spatial)
+    out["attention_function_name"] = ba.attention_function.__name__
+    q = torch.randn(2, 16, 128, generator=torch.Generator().manual_seed(15))
+    out["deferred_q"], out["deferred_out"] = q, ba.attention_function(q, q, q, 2)
+
+    def record_attention(mod, model, inputs):
+        """The first call of each distinct signature; replayed on seeded inputs of the same shapes (what is stored is the
+        seed and a seeded sample of the reference's output)."""
+        seen, calls = set(), []
+        orig = mod.attention_function
+
+        def rec(q, k, v, heads, *a, **kw):
+            sig = (tuple(q.shape), tuple(k.shape), tuple(v.shape), heads, a, tuple(sorted(kw.items())))
+            if sig not in seen:
+                seen.add(sig)
+                calls.append(sig)
+            return orig(q, k, v, heads, *a, **kw)
+        mod.attention_function = rec
+        try:
+            with torch.no_grad():
+                model(*inputs[0], **inputs[1])
+        finally:
+            mod.attention_function = orig
+        out = []
+        for i, (qs, ks, vs, heads, a, kw) in enumerate(calls):
+            seed = 100 + i
+            q, k, v = seeded_inputs((qs, ks, vs), seed)
+            with torch.no_grad():
+                o = orig(q, k, v, heads, *a, **dict(kw))
+            idx = sample_index(o.numel(), seed)
+            out.append(dict(shapes=(qs, ks, vs), heads=heads, args=a, kwargs=dict(kw), seed=seed, out_shape=tuple(o.shape),
+                            out_sample=o.reshape(-1)[idx].clone()))
+        return out
+
+    g = torch.load(os.path.join(GOLD, "unet_tiny_xl.pt"), weights_only=False)
+    cfg = CF.CONFIGS["tiny_xl"]
+    m = bu.IntegratedUNet2DConditionModel(**cfg).eval()
+    m.load_state_dict(OU.random_state_dict(cfg, seed=g["weight_seed"]), strict=True)
+    out["unet_attention_calls"] = record_attention(bu, m, ((g["x"], g["t"]), dict(context=g["context"], y=g["y"], transformer_options={})))
+    gf = torch.load(os.path.join(GOLD, "flux_tiny.pt"), weights_only=False)
+    fcfg = OF.CONFIGS[gf["config"]]
+    fm = bf.IntegratedFluxTransformer2DModel(**fcfg).eval()
+    fm.load_state_dict(OF.random_state_dict(fcfg, seed=gf["weight_seed"]), strict=True)
+    out["flux_attention_calls"] = record_attention(bf, fm, ((gf["x"], gf["t"], gf["context"], gf["y"], gf["guidance"]), {}))
+    print("attention calls recorded", len(out["unet_attention_calls"]), len(out["flux_attention_calls"]), out["attention_importers"])
+
+    # P3, UNet
+    sd = OU.random_state_dict(cfg, seed=1)
+    unet = bu.IntegratedUNet2DConditionModel(**cfg).eval()
+    unet.load_state_dict(sd, strict=True)
+    unet.storage_dtype = unet.computation_dtype = torch.float32
+    kmodel = KModel(unet, diffusers_scheduler=None, k_predictor=Prediction(prediction_type="epsilon"))
+    g = torch.Generator().manual_seed(3)
+    B = 2
+    cond = dict(crossattn=torch.randn(B, 77, cfg["context_dim"], generator=g), vector=torch.randn(B, cfg["adm_in_channels"], generator=g))
+    uncond = dict(crossattn=torch.randn(B, 77, cfg["context_dim"], generator=g), vector=torch.randn(B, cfg["adm_in_channels"], generator=g))
+    x = torch.randn(B, 4, 16, 16, generator=g) * 4
+    out["p3_unet"] = dict(config="tiny_xl", weight_seed=1,
+                          **_record_wrapper_call(kmodel, x, torch.tensor([6.0, 6.0]), compile_conditions(uncond), compile_conditions(cond), 7.0))
+    # P3, Flux
+    fcfg = OF.TINY_FLUX
+    fsd = OF.random_state_dict(fcfg, seed=5)
+    fm = bf.IntegratedFluxTransformer2DModel(**fcfg).eval()
+    fm.load_state_dict(fsd, strict=True)
+    fm.storage_dtype = fm.computation_dtype = torch.float32
+    kmodel = KModel(fm, diffusers_scheduler=None, k_predictor=PredictionFlux())
+    g = torch.Generator().manual_seed(6)
+    cond = dict(crossattn=torch.randn(B, 64, fcfg["context_in_dim"], generator=g), vector=torch.randn(B, fcfg["vec_in_dim"], generator=g),
+                guidance=torch.full((B,), 4.0))
+    x = torch.randn(B, 16, 16, 16, generator=g)
+    out["p3_flux"] = dict(config="tiny_flux", weight_seed=5,
+                          **_record_wrapper_call(kmodel, x, torch.tensor([0.8, 0.8]), None, compile_conditions(cond), 1.0))
+    for k in ("p3_unet", "p3_flux"):
+        print(k, {a: (tuple(v.shape) if torch.is_tensor(v) else v) for a, v in out[k]["args"]["c"].items()})
+    torch.save(out, os.path.join(GOLD, "plugin_calls.pt"))
+
+
+def gen_module_calls():
+    """P2: every Linear / Conv2d / GroupNorm / LayerNorm module the reference UNet (tiny_xl), VAE decoder (tiny) and Flux
+    transformer (tiny) run in the forwards of unet_tiny_xl.pt / vae_tiny.pt / flux_tiny.pt — its constructor arguments,
+    state-dict name and input shape; the first module of each distinct (constructor, input shape) is run once more on a
+    seeded input of that shape and a seeded sample of its output is stored."""
+    from backend.nn.flux import IntegratedFluxTransformer2DModel
+    from backend.nn.unet import IntegratedUNet2DConditionModel as RefUNet
+    from backend.nn.vae import IntegratedAutoencoderKL
+    from oracle import flux as OF
+    from oracle import vae as OV
+    nn = torch.nn
+
+    def ctor(mod):
+        if isinstance(mod, nn.Linear):
+            return "Linear", dict(in_features=mod.in_features, out_features=mod.out_features, bias=mod.bias is not None)
+        if isinstance(mod, nn.Conv2d):
+            return "Conv2d", dict(in_channels=mod.in_channels, out_channels=mod.out_channels, kernel_size=mod.kernel_size,
+                                  stride=mod.stride, padding=mod.padding, bias=mod.bias is not None)
+        if isinstance(mod, nn.GroupNorm):
+            return "GroupNorm", dict(num_groups=mod.num_groups, num_channels=mod.num_channels, eps=mod.eps, affine=mod.affine)
+        if isinstance(mod, nn.LayerNorm):
+            return "LayerNorm", dict(normalized_shape=tuple(mod.normalized_shape), eps=mod.eps, elementwise_affine=mod.elementwise_affine)
+        return None
+
+    def record(model, run):
+        calls, seen, hooks = [], set(), []
+        for name, mod in model.named_modules():
+            c = ctor(mod)
+            if c is None:
+                continue
+
+            def hook(m, inp, o, name=name, c=c):
+                sig = (c[0], tuple(sorted(c[1].items())), tuple(inp[0].shape))
+                entry = dict(name=name, kind=c[0], kwargs=c[1], x_shape=tuple(inp[0].shape))
+                if sig not in seen:
+                    seen.add(sig)
+                    entry["replay"] = m
+                calls.append(entry)
+            hooks.append(mod.register_forward_hook(hook))
+        try:
+            with torch.no_grad():
+                run()
+        finally:
+            for h in hooks:
+                h.remove()
+        for i, entry in enumerate(c for c in calls if "replay" in c):
+            mod = entry.pop("replay")
+            seed = 200 + i
+            x, = seeded_inputs((entry["x_shape"],), seed)
+            with torch.no_grad():
+                o = mod(x)
+            idx = sample_index(o.numel(), seed)
+            entry.update(seed=seed, out_shape=tuple(o.shape), out_sample=o.reshape(-1)[idx].clone())
+        return calls
+
+    out = {}
+    g = torch.load(os.path.join(GOLD, "unet_tiny_xl.pt"), weights_only=False)
+    cfg = CF.CONFIGS[g["config"]]
+    m = RefUNet(**cfg).eval()
+    m.load_state_dict(OU.random_state_dict(cfg, seed=g["weight_seed"]), strict=True)
+    out["unet"] = dict(config=g["config"], weight_seed=g["weight_seed"],
+                       calls=record(m, lambda: m(g["x"], g["t"], context=g["context"], y=g["y"], transformer_options={})))
+    gv = torch.load(os.path.join(GOLD, "vae_tiny.pt"), weights_only=False)
+    vcfg = CF.VAE_CONFIGS[gv["config"]]
+    vae = IntegratedAutoencoderKL(**vcfg).eval()
+    vae.load_state_dict(OV.random_state_dict(vcfg, seed=gv["weight_seed"]), strict=False)
+    out["vae"] = dict(config=gv["config"], weight_seed=gv["weight_seed"], calls=record(vae, lambda: vae.decode(vae.process_out(gv["z"]))))
+    gf = torch.load(os.path.join(GOLD, "flux_tiny.pt"), weights_only=False)
+    fcfg = OF.CONFIGS[gf["config"]]
+    fm = IntegratedFluxTransformer2DModel(**fcfg).eval()
+    fm.load_state_dict(OF.random_state_dict(fcfg, seed=gf["weight_seed"]), strict=True)
+    out["flux"] = dict(config=gf["config"], weight_seed=gf["weight_seed"],
+                       calls=record(fm, lambda: fm(gf["x"], gf["t"], gf["context"], gf["y"], gf["guidance"])))
+    for k, v in out.items():
+        kinds = {}
+        for c in v["calls"]:
+            kinds[c["kind"]] = kinds.get(c["kind"], 0) + 1
+        print("module calls", k, kinds, "replayed:", sum(1 for c in v["calls"] if "seed" in c))
+    torch.save(out, os.path.join(GOLD, "module_calls.pt"))
+
+
 if __name__ == "__main__":
     os.makedirs(GOLD, exist_ok=True)
     ref_import.load()
-    which = sys.argv[1:] or ["unet", "traj", "vtraj", "sched", "samplers", "vae", "vae_tiled", "vae_enc", "control", "chroma", "flux", "flux_odd"]
+    which = sys.argv[1:] or ["unet", "traj", "vtraj", "sched", "samplers", "vae", "vae_tiled", "vae_enc", "control", "chroma", "flux", "flux_odd",
+                             "unet_b1", "param_shapes", "plugin_calls", "module_calls"]
     if "unet" in which:
         gen_unet("tiny_xl")
         gen_unet("tiny_15")
@@ -464,3 +709,11 @@ if __name__ == "__main__":
         gen_flux(hw=32, txt_len=256, fname="flux_tiny_seg.pt")      # 256 + 256 tokens: two-segment GEMM path
     if "flux_odd" in which:
         gen_flux(hw=15, hw_w=18, txt_len=64, fname="flux_tiny_odd.pt")  # odd height: circular pad to the patch size + crop
+    if "unet_b1" in which:
+        gen_unet_b1()
+    if "param_shapes" in which:
+        gen_param_shapes()
+    if "plugin_calls" in which:
+        gen_plugin_calls()
+    if "module_calls" in which:
+        gen_module_calls()

@@ -197,26 +197,31 @@ def unet_forward(sd: SD, cfg: dict, x, timesteps, context, y: Optional[torch.Ten
     return h.type(x.dtype)
 
 
-def random_state_dict(cfg: dict, seed: int = 0, dtype=torch.float32) -> SD:
+def random_state_dict(cfg: dict, seed: int = 0, dtype=torch.float32, device=None) -> SD:
     """Deterministic synthetic weights with the reference's parameter names and shapes.
     ForgeOperations.*.reset_parameters are no-ops (backend/operations.py:166-167), so there is no reference
     initialisation to mirror; weights are N(0, 1/fan_in)-scaled so activations stay O(1) through the net,
     norm gains ~ 1, biases small."""
     g = torch.Generator().manual_seed(seed)
+    assert device in (None, "cpu", "meta"), device
+
+    def randn(*shape):  # device="meta": names and shapes only, nothing drawn or allocated
+        return torch.empty(*shape, device="meta") if device == "meta" else torch.randn(*shape, generator=g)
+
     sd: SD = {}
 
     def lin(p, cin, cout, bias=True):
-        sd[p + ".weight"] = (torch.randn(cout, cin, generator=g) * cin ** -0.5).to(dtype)
+        sd[p + ".weight"] = (randn(cout, cin) * cin ** -0.5).to(dtype)
         if bias:
-            sd[p + ".bias"] = (torch.randn(cout, generator=g) * 0.05).to(dtype)
+            sd[p + ".bias"] = (randn(cout) * 0.05).to(dtype)
 
     def conv(p, cin, cout, k):
-        sd[p + ".weight"] = (torch.randn(cout, cin, k, k, generator=g) * (cin * k * k) ** -0.5).to(dtype)
-        sd[p + ".bias"] = (torch.randn(cout, generator=g) * 0.05).to(dtype)
+        sd[p + ".weight"] = (randn(cout, cin, k, k) * (cin * k * k) ** -0.5).to(dtype)
+        sd[p + ".bias"] = (randn(cout) * 0.05).to(dtype)
 
     def norm(p, c):
-        sd[p + ".weight"] = (1.0 + 0.1 * torch.randn(c, generator=g)).to(dtype)
-        sd[p + ".bias"] = (0.05 * torch.randn(c, generator=g)).to(dtype)
+        sd[p + ".weight"] = (1.0 + 0.1 * randn(c)).to(dtype)
+        sd[p + ".bias"] = (0.05 * randn(c)).to(dtype)
 
     mc = cfg["model_channels"]
     ted = mc * 4

@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
 import threading
 
@@ -134,7 +135,10 @@ _lock = threading.Lock()
 
 def build(verbose: bool = False) -> str:
     """Compile csrc/*.cu for sm_100a into libb200forge.so (nvcc cross-compiles without a GPU)."""
-    r = subprocess.run(["make", "-C", CSRC_DIR, "-j8"], capture_output=True, text=True)
+    cmd = ["make", "-C", CSRC_DIR, "-j8"]
+    if shutil.which("nvcc") is None:  # a CUDA install that is not on PATH
+        cmd.append("NVCC=" + os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc"))
+    r = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or r.returncode != 0:
         print(r.stdout[-4000:])
         print(r.stderr[-4000:])

@@ -3,7 +3,8 @@ replaced by its torch emulation (tests/ops_emulator.py) and the engines run in f
 reference goldens (tests/golden, made by the imported reference) to ~1e-4 — far tighter than the fp16/bf16 tolerances of the
 GPU parity tests, which is what exposes packing / folding / ordering mistakes.  The CUDA kernels themselves are NOT
 exercised here (that is what `-m gpu` does through the C ABI)."""
-import os
+import sys
+import types
 
 import pytest
 import torch
@@ -13,15 +14,15 @@ from oracle import flux as OF
 from oracle import sampling as S
 from oracle import unet as OU
 from oracle import vae as OV
+from oracle.golden import load_golden, sample_index, seeded_inputs
 from tests import ops_emulator
 from tests.util import assert_close
 
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 F32 = torch.float32
 
 
 def _gold(name):
-    return torch.load(os.path.join(GOLD, name), weights_only=False)
+    return load_golden(name)
 
 
 @pytest.fixture(autouse=True)
@@ -123,89 +124,63 @@ def test_v_prediction_pipeline_host_logic_vs_reference_trajectory():
 
 
 # --------------------------------------------------------------------------------------------------------------------
-# Plug point P3 wired into the UNMODIFIED reference: backend.sampling.sampling_function.sampling_function_inner calls
-# model_options['model_function_wrapper'] (sampling_function.py:270-273) exactly as Forge does; with the wrapper installed
-# the result must equal the reference's own apply_model path.  (CPU: the engine runs on the emulated ops.)
-from oracle import ref_import  # noqa: E402
+# Plug points against what the UNMODIFIED reference hands them (tests/golden/plugin_calls.pt, module_calls.pt, recorded by
+# oracle/gen_golden.py): P3 gets the exact argument dict backend.sampling.sampling_function.sampling_function_inner passes to
+# model_options['model_function_wrapper'] (sampling_function.py:270-273) and must return what the reference's own
+# apply_model returned for it; P1 / P2 get the reference models' attention calls and operator modules.  (CPU: the engines
+# and operators run on the emulated ops.)
+class _RecordedPredictor:
+    """The reference predictor of a recorded P3 call: its prediction type, and timestep() as it evaluated for that call."""
+
+    def __init__(self, rec):
+        self.prediction_type, self._sigma, self._t = rec["prediction_type"], rec["args"]["timestep"], rec["timestep_from_sigma"]
+
+    def timestep(self, sigma):
+        assert torch.equal(sigma, self._sigma)
+        return self._t
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
+def _reference_apply_model(*a, **kw):
+    raise AssertionError("the wrapper handed the call back to the reference's apply_model")
+
+
 def test_p3_unet_wrapper_inside_the_reference_sampling_function(monkeypatch):
-    ref_import.load()
-    from backend.modules.k_model import KModel
-    from backend.modules.k_prediction import Prediction
-    from backend.nn.unet import IntegratedUNet2DConditionModel as RefUNet
-    from backend.sampling.condition import compile_conditions
-    from backend.sampling.sampling_function import sampling_function_inner
-
     from b200forge import plugin
     from b200forge.unet_engine import UNetEngine
     monkeypatch.setattr(plugin, "_on_device", lambda t: True)
-    cfg = CF.CONFIGS["tiny_xl"]
-    sd = OU.random_state_dict(cfg, seed=1)
-    unet = RefUNet(**cfg).eval()
-    unet.load_state_dict(sd, strict=True)
-    unet.storage_dtype = unet.computation_dtype = torch.float32
-    kmodel = KModel(unet, diffusers_scheduler=None, k_predictor=Prediction(prediction_type="epsilon"))
-    g = torch.Generator().manual_seed(3)
-    B = 2
-    cond = dict(crossattn=torch.randn(B, 77, cfg["context_dim"], generator=g), vector=torch.randn(B, cfg["adm_in_channels"], generator=g))
-    uncond = dict(crossattn=torch.randn(B, 77, cfg["context_dim"], generator=g), vector=torch.randn(B, cfg["adm_in_channels"], generator=g))
-    cc, uc = compile_conditions(cond), compile_conditions(uncond)
-    x = torch.randn(B, 4, 16, 16, generator=g) * 4
-    sigma = torch.tensor([6.0, 6.0])
+    rec = _gold("plugin_calls.pt")["p3_unet"]
+    cfg = CF.CONFIGS[rec["config"]]
+    w = plugin.UNetWrapper(UNetEngine(cfg, OU.random_state_dict(cfg, seed=rec["weight_seed"]), dtype=F32, device="cpu"),
+                           _RecordedPredictor(rec))
     with torch.no_grad():
-        base = sampling_function_inner(kmodel, x, sigma, uc, cc, 7.0, {}, None)
-        w = plugin.UNetWrapper(UNetEngine(cfg, sd, dtype=F32, device="cpu"), kmodel.predictor)
-        out = sampling_function_inner(kmodel, x, sigma, uc, cc, 7.0, {"model_function_wrapper": w}, None)
+        out = w(_reference_apply_model, rec["args"])
     assert w.calls_fast == 1 and w.calls_reference == 0
-    assert_close("reference sampling_function with the fused UNet wrapper vs without", out, base, rel_rms=1e-5)
+    assert_close("fused UNet wrapper vs the reference's apply_model for the same call", out, rec["out"], rel_rms=1e-5)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
 def test_p3_flux_wrapper_inside_the_reference_sampling_function(monkeypatch):
-    ref_import.load()
-    from backend.modules.k_model import KModel
-    from backend.modules.k_prediction import PredictionFlux
-    from backend.nn.flux import IntegratedFluxTransformer2DModel
-    from backend.sampling.condition import compile_conditions
-    from backend.sampling.sampling_function import sampling_function_inner
-
     from b200forge import plugin
     from b200forge.flux_engine import FluxEngine
     monkeypatch.setattr(plugin, "_on_device", lambda t: True)
-    cfg = OF.TINY_FLUX
-    sd = OF.random_state_dict(cfg, seed=5)
-    m = IntegratedFluxTransformer2DModel(**cfg).eval()
-    m.load_state_dict(sd, strict=True)
-    m.storage_dtype = m.computation_dtype = torch.float32
-    kmodel = KModel(m, diffusers_scheduler=None, k_predictor=PredictionFlux())
-    g = torch.Generator().manual_seed(6)
-    B = 2
-    cond = dict(crossattn=torch.randn(B, 64, cfg["context_in_dim"], generator=g), vector=torch.randn(B, cfg["vec_in_dim"], generator=g),
-                guidance=torch.full((B,), 4.0))
-    cc = compile_conditions(cond)
-    x = torch.randn(B, 16, 16, 16, generator=g)
-    sigma = torch.tensor([0.8, 0.8])
+    rec = _gold("plugin_calls.pt")["p3_flux"]
+    cfg = OF.CONFIGS[rec["config"]]
+    w = plugin.FluxWrapper(FluxEngine(cfg, OF.random_state_dict(cfg, seed=rec["weight_seed"]), dtype=F32, device="cpu"),
+                           _RecordedPredictor(rec))
     with torch.no_grad():
-        base = sampling_function_inner(kmodel, x, sigma, None, cc, 1.0, {}, None)
-        w = plugin.FluxWrapper(FluxEngine(cfg, sd, dtype=F32, device="cpu"), kmodel.predictor)
-        out = sampling_function_inner(kmodel, x, sigma, None, cc, 1.0, {"model_function_wrapper": w}, None)
+        out = w(_reference_apply_model, rec["args"])
     assert w.calls_fast == 1 and w.calls_reference == 0
-    assert_close("reference sampling_function with the fused Flux wrapper vs without", out, base, rel_rms=1e-5)
+    assert_close("fused Flux wrapper vs the reference's apply_model for the same call", out, rec["out"], rel_rms=1e-5)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
 def test_p1_attention_operator_inside_the_reference_models(monkeypatch):
     """plugin.install_attention() rebinds the by-value imports of attention_function in the reference's model files
-    (backend/nn/unet.py:5, flux.py:11); the reference UNet (Dh = 64, [b, L, H*Dh] layout) and Flux transformer (Dh = 128,
-    skip_reshape layout) then call the B200 operator and must reproduce their goldens.  (CPU: the operator's kernels are the emulated ops; the device / dtype gate is opened for the test.)"""
-    ref_import.load()
-    from backend.nn.flux import IntegratedFluxTransformer2DModel
-    from backend.nn.unet import IntegratedUNet2DConditionModel as RefUNet
-
+    (backend/nn/unet.py:5, flux.py:11); every distinct attention call the reference UNet (Dh = 64, [b, L, H*Dh] layout) and
+    Flux transformer (Dh = 128, skip_reshape layout) make, replayed through the rebound names on seeded inputs of the same
+    shapes, must run the B200 operator and reproduce the reference's result.  (CPU: the operator's kernels are the emulated
+    ops; the device / dtype gate is opened for the test.)"""
     from b200forge import attention as A
-    from b200forge import plugin
+    from b200forge import ops, plugin
+    rec = _gold("plugin_calls.pt")
     calls = {"n": 0}
     real_attn, real_single = A.attention_function, A.attention_function_single_head_spatial
 
@@ -219,65 +194,84 @@ def test_p1_attention_operator_inside_the_reference_models(monkeypatch):
         calls["n"] += 1
         return orig_attention(*a, **kw)
 
-    from b200forge import ops
     monkeypatch.setattr(ops, "attention", counting_attention)
+
+    def attention_pytorch(*a, **kw):
+        raise AssertionError("deferred to the reference attention")
+
+    for name in ["backend.attention"] + rec["attention_importers"]:
+        monkeypatch.setitem(sys.modules, name, types.ModuleType(name))
+        sys.modules[name].attention_function = attention_pytorch
+    sys.modules["backend.attention"].attention_function_single_head_spatial = attention_pytorch
     plugin.install_attention()
     try:
-        g = _gold("unet_tiny_xl.pt")
-        cfg = CF.CONFIGS["tiny_xl"]
-        m = RefUNet(**cfg).eval()
-        m.load_state_dict(OU.random_state_dict(cfg, seed=g["weight_seed"]), strict=True)
-        with torch.no_grad():
-            out = m(g["x"], g["t"], context=g["context"], y=g["y"], transformer_options={})
-        assert calls["n"] > 0
-        assert_close("reference UNet calling the B200 attention operator", out, g["out"], max_abs=5e-5)
-        n_unet = calls["n"]
-        gf = _gold("flux_tiny.pt")
-        fcfg = OF.CONFIGS[gf["config"]]
-        fm = IntegratedFluxTransformer2DModel(**fcfg).eval()
-        fm.load_state_dict(OF.random_state_dict(fcfg, seed=gf["weight_seed"]), strict=True)
-        with torch.no_grad():
-            fout = fm(gf["x"], gf["t"], gf["context"], gf["y"], gf["guidance"])
-        assert calls["n"] > n_unet
-        assert_close("reference Flux transformer calling the B200 attention operator", fout, gf["out"], max_abs=5e-5)
+        for key, module in (("unet_attention_calls", "backend.nn.unet"), ("flux_attention_calls", "backend.nn.flux")):
+            fn = sys.modules[module].attention_function
+            assert fn is A.attention_function and rec[key]
+            for c in rec[key]:
+                q, k, v = seeded_inputs(c["shapes"], c["seed"])
+                n0 = calls["n"]
+                with torch.no_grad():
+                    out = fn(q, k, v, c["heads"], *c["args"], **c["kwargs"])
+                assert calls["n"] == n0 + 1 and tuple(out.shape) == c["out_shape"]
+                assert_close(f"reference {module} attention call {c['shapes']} through the B200 operator",
+                             out.reshape(-1)[sample_index(out.numel(), c["seed"])], c["out_sample"], max_abs=5e-5)
     finally:
         plugin.uninstall_attention()
     assert A.attention_function is real_attn and A.attention_function_single_head_spatial is real_single
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
+def _replay_module_calls(model, state_dict):
+    """Build each distinct operator module the reference model runs from B200Operations with the reference's constructor
+    arguments and weights, and run it on a seeded input of the recorded shape: it must reproduce the reference module's
+    output.  Returns the module kinds seen in the whole recorded forward."""
+    from b200forge import operations as P2
+    rec = _gold("module_calls.pt")[model]
+    kinds = set()
+    for c in rec["calls"]:
+        kinds.add(c["kind"])
+        mod = getattr(P2.B200Operations, c["kind"])(**c["kwargs"])
+        own = {k[len(c["name"]) + 1:]: v for k, v in state_dict.items() if k.startswith(c["name"] + ".")}
+        mod.load_state_dict(own, strict=True)  # the oracle state dict names every parameter of every recorded module
+        if "seed" not in c:
+            continue
+        x, = seeded_inputs((c["x_shape"],), c["seed"])
+        with torch.no_grad():
+            out = mod(x)
+        assert tuple(out.shape) == c["out_shape"]
+        assert_close(f"{model} {c['name']} ({c['kind']}) built from B200Operations",
+                     out.reshape(-1)[sample_index(out.numel(), c["seed"])], c["out_sample"], max_abs=5e-5)
+    return kinds
+
+
+def _count_ops(monkeypatch, names):
+    from b200forge import ops
+    counted = dict.fromkeys(names, 0)
+    for name in names:
+        fn = getattr(ops, name)
+
+        def wrap(*a, _fn=fn, _k=name, **kw):
+            counted[_k] += 1
+            return _fn(*a, **kw)
+        monkeypatch.setattr(ops, name, wrap)
+    return counted
+
+
 def test_p2_operator_classes_inside_the_reference_unet(monkeypatch):
     """backend.operations.using_forge_operations(operations=B200Operations) (backend/operations.py:441-467): the
     reference constructs its UNet from our Linear / Conv2d / GroupNorm / LayerNorm modules.  Their NCHW / [.., C] boundary
     conversions and routing (3x3 stride 1 -> implicit GEMM, stride 2 -> im2col + GEMM, 1x1 -> GEMM) must reproduce the
-    golden.  (CPU: emulated kernels, device / dtype gate opened for the test.)"""
-    ref_import.load()
-    from backend.nn.unet import IntegratedUNet2DConditionModel as RefUNet
-    from backend.operations import using_forge_operations
-
+    reference's modules, each built with the reference's constructor arguments.  (CPU: emulated kernels, device / dtype
+    gate opened for the test.)"""
     from b200forge import operations as P2
     monkeypatch.setattr(P2, "_fast", lambda x, w: w.dtype == x.dtype)
     monkeypatch.setattr(P2, "DEFERRED", 0)
-    g = _gold("unet_tiny_xl.pt")
-    cfg = CF.CONFIGS["tiny_xl"]
-    with using_forge_operations(operations=P2.B200Operations, device=torch.device("cpu"), dtype=torch.float32):
-        m = RefUNet(**cfg).eval()
-    kinds = {type(mod) for mod in m.modules()}
-    assert P2.Linear in kinds and P2.Conv2d in kinds and P2.GroupNorm in kinds and P2.LayerNorm in kinds
-    m.load_state_dict(OU.random_state_dict(cfg, seed=g["weight_seed"]), strict=True)
-    counted = {"gemm": 0, "conv": 0, "gn": 0}
-    from b200forge import ops
-    for name, key in (("gemm", "gemm"), ("conv3x3", "conv"), ("groupnorm", "gn")):
-        fn = getattr(ops, name)
-
-        def wrap(*a, _fn=fn, _k=key, **kw):
-            counted[_k] += 1
-            return _fn(*a, **kw)
-        monkeypatch.setattr(ops, name, wrap)
-    with torch.no_grad():
-        out = m(g["x"], g["t"], context=g["context"], y=g["y"], transformer_options={})
-    assert counted["gemm"] > 50 and counted["conv"] > 20 and counted["gn"] > 20, counted
-    assert_close("reference UNet built from B200Operations modules", out, g["out"], max_abs=5e-5)
+    counted = _count_ops(monkeypatch, ["gemm", "conv3x3_any", "im2col3x3", "groupnorm"])
+    rec = _gold("module_calls.pt")["unet"]
+    cfg = CF.CONFIGS[rec["config"]]
+    kinds = _replay_module_calls("unet", OU.random_state_dict(cfg, seed=rec["weight_seed"]))
+    assert kinds == {"Linear", "Conv2d", "GroupNorm", "LayerNorm"}
+    assert all(counted.values()), counted
 
 
 def test_hires_fix_host_logic_vs_oracle_composition():
@@ -372,33 +366,16 @@ def test_unet_engine_control_residuals_vs_reference_golden(monkeypatch):
     assert_close("P3 wrapper with control vs oracle", den, pred.calculate_denoised(sigma, eps, x), rel_rms=1e-5)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
 def test_p2_operator_classes_inside_the_reference_vae_and_flux(monkeypatch):
     """Same as above for the reference VAE decoder (Conv2d / GroupNorm at 3 and 4-channel edges, 1x1 attention convs) and
     the Flux transformer (Linear everywhere, LayerNorm without affine) built from B200Operations."""
-    ref_import.load()
-    from backend.nn.flux import IntegratedFluxTransformer2DModel
-    from backend.nn.vae import IntegratedAutoencoderKL
-    from backend.operations import using_forge_operations
-
     from b200forge import operations as P2
     monkeypatch.setattr(P2, "_fast", lambda x, w: w.dtype == x.dtype)
     monkeypatch.setattr(P2, "_FAST_DTYPES", (torch.float16, torch.bfloat16, torch.float32))
-    gv = _gold("vae_tiny.pt")
-    vcfg = CF.VAE_CONFIGS[gv["config"]]
-    with using_forge_operations(operations=P2.B200Operations, device=torch.device("cpu"), dtype=torch.float32):
-        vae = IntegratedAutoencoderKL(**vcfg).eval()
-        gf = _gold("flux_tiny.pt")
-        fcfg = OF.CONFIGS[gf["config"]]
-        flux = IntegratedFluxTransformer2DModel(**fcfg).eval()
-    assert any(isinstance(m, P2.Conv2d) for m in vae.modules()) and any(isinstance(m, P2.Linear) for m in flux.modules())
-    vae.load_state_dict(OV.random_state_dict(vcfg, seed=gv["weight_seed"]), strict=False)
-    flux.load_state_dict(OF.random_state_dict(fcfg, seed=gf["weight_seed"]), strict=True)
-    with torch.no_grad():
-        img = vae.decode(vae.process_out(gv["z"]))
-        out = flux(gf["x"], gf["t"], gf["context"], gf["y"], gf["guidance"])
-    assert_close("reference VAE decoder built from B200Operations modules", img, gv["out"], max_abs=5e-5)
-    assert_close("reference Flux transformer built from B200Operations modules", out, gf["out"], max_abs=5e-5)
+    rv, rf = _gold("module_calls.pt")["vae"], _gold("module_calls.pt")["flux"]
+    vcfg, fcfg = CF.VAE_CONFIGS[rv["config"]], OF.CONFIGS[rf["config"]]
+    assert _replay_module_calls("vae", OV.random_state_dict(vcfg, seed=rv["weight_seed"])) == {"Conv2d", "GroupNorm"}
+    assert "Linear" in _replay_module_calls("flux", OF.random_state_dict(fcfg, seed=rf["weight_seed"]))
 
 
 def test_flux_img2img_host_logic_vs_oracle_loop():
@@ -545,13 +522,107 @@ def test_p3_wrapper_follows_lora_refresh(monkeypatch):
     assert_close("P3 wrapper after the LoRA was removed", call(), base, rel_rms=1e-6)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
-def test_p2_installed_operations_subclass_forges_own_classes():
+def _forge_operations_module():
+    """A stand-in for backend.operations with the behaviour of Forge's operator set that the B200 classes must keep when
+    they subclass it (backend/operations.py:119-167, 442-467): Linear creates no weight until its state dict is loaded (a
+    `dummy` parameter carries the storage device / dtype); every class records `parameters_manual_cast` at construction and
+    then computes in the input's dtype from weights stored in another one; using_forge_operations() swaps the torch.nn
+    classes for the operator set's, which is looked up as `ForgeOperations` at call time.  Each forward of the stand-in
+    counts itself, so a call that reached the parent can be told apart from one the B200 class served."""
+    import contextlib
+
+    F = torch.nn.functional
+    bo = types.ModuleType("backend.operations")
+    bo.current_device = bo.current_dtype = None
+    bo.current_manual_cast_enabled = False
+    bo.parent_forwards = 0
+
+    def cast(mod, x):
+        bo.parent_forwards += 1
+        if not mod.parameters_manual_cast:
+            return mod.weight, mod.bias
+        return mod.weight.to(x.dtype), None if mod.bias is None else mod.bias.to(x.dtype)
+
+    class Linear(torch.nn.Module):
+        def __init__(self, in_features, out_features, *args, **kwargs):
+            super().__init__()
+            self.in_features, self.out_features = in_features, out_features
+            self.dummy = torch.nn.Parameter(torch.empty(1, device=bo.current_device, dtype=bo.current_dtype))
+            self.weight = self.bias = None
+            self.parameters_manual_cast = bo.current_manual_cast_enabled
+
+        def _load_from_state_dict(self, state_dict, prefix, *args):
+            if not hasattr(self, "dummy"):
+                return super()._load_from_state_dict(state_dict, prefix, *args)
+            for name in ("weight", "bias"):
+                if prefix + name in state_dict:
+                    setattr(self, name, torch.nn.Parameter(state_dict[prefix + name].to(self.dummy)))
+            del self.dummy
+
+        def forward(self, x):
+            return F.linear(x, *cast(self, x))
+
+    def storage_kwargs(kwargs):
+        return dict(kwargs, device=bo.current_device, dtype=bo.current_dtype)
+
+    class Conv2d(torch.nn.Conv2d):
+        def __init__(self, *args, **kwargs):
+            super().__init__(*args, **storage_kwargs(kwargs))
+            self.parameters_manual_cast = bo.current_manual_cast_enabled
+
+        def reset_parameters(self):
+            return None
+
+        def forward(self, x):
+            return self._conv_forward(x, *cast(self, x))
+
+    class GroupNorm(torch.nn.GroupNorm):
+        def __init__(self, *args, **kwargs):
+            super().__init__(*args, **storage_kwargs(kwargs))
+            self.parameters_manual_cast = bo.current_manual_cast_enabled
+
+        def forward(self, x):
+            return F.group_norm(x, self.num_groups, *cast(self, x), self.eps)
+
+    class LayerNorm(torch.nn.LayerNorm):
+        def __init__(self, *args, **kwargs):
+            super().__init__(*args, **storage_kwargs(kwargs))
+            self.parameters_manual_cast = bo.current_manual_cast_enabled
+
+        def forward(self, x):
+            return F.layer_norm(x, self.normalized_shape, *cast(self, x), self.eps)
+
+    class Embedding(torch.nn.Embedding):
+        pass
+
+    bo.ForgeOperations = type("ForgeOperations", (), dict(Linear=Linear, Conv2d=Conv2d, GroupNorm=GroupNorm, LayerNorm=LayerNorm,
+                                                          Embedding=Embedding))
+    names = ("Linear", "Conv2d", "GroupNorm", "LayerNorm", "Embedding")
+
+    @contextlib.contextmanager
+    def using_forge_operations(operations=None, device=None, dtype=None, manual_cast_enabled=False):
+        bo.current_device, bo.current_dtype, bo.current_manual_cast_enabled = device, dtype, manual_cast_enabled
+        operations = bo.ForgeOperations if operations is None else operations
+        saved = {n: getattr(torch.nn, n) for n in names}
+        try:
+            for n in names:
+                setattr(torch.nn, n, getattr(operations, n))
+            yield
+        finally:
+            for n, cls in saved.items():
+                setattr(torch.nn, n, cls)
+
+    bo.using_forge_operations = using_forge_operations
+    return bo
+
+
+def test_p2_installed_operations_subclass_forges_own_classes(monkeypatch):
     """plugin.install_operations(): the hot-path classes SUBCLASS ForgeOperations' classes, so lazy weights
     (`dummy` / `_load_from_state_dict`), `parameters_manual_cast` (storage dtype != computation dtype: fp8 / bf16 storage) and
-    `forge_online_loras` keep the reference's behaviour — such calls run the parent's forward (backend/operations.py:126-156)."""
-    ref_import.load()
-    import backend.operations as bo
+    `forge_online_loras` keep the reference's behaviour — such calls run the parent's forward (backend/operations.py:126-156).
+    Forge's operator set is the stand-in above."""
+    bo = _forge_operations_module()
+    monkeypatch.setitem(sys.modules, "backend.operations", bo)
 
     from b200forge import operations as B, plugin
     forge = bo.ForgeOperations
@@ -562,18 +633,22 @@ def test_p2_installed_operations_subclass_forges_own_classes():
         with bo.using_forge_operations(device="cpu", dtype=torch.bfloat16, manual_cast_enabled=True):
             lin = torch.nn.Linear(16, 32)
             conv = torch.nn.Conv2d(8, 16, 3, padding=1)
+        assert type(lin) is bo.ForgeOperations.Linear and type(conv) is bo.ForgeOperations.Conv2d
         assert isinstance(lin, forge.Linear) and lin.parameters_manual_cast and lin.weight is None  # Forge's lazy init
         g = torch.Generator().manual_seed(0)
         wl, bl = torch.randn(32, 16, generator=g).bfloat16(), torch.randn(32, generator=g).bfloat16()
         lin.load_state_dict({"weight": wl, "bias": bl})
+        assert lin.weight.dtype == torch.bfloat16 and not hasattr(lin, "dummy")
         conv.load_state_dict({"weight": torch.randn(16, 8, 3, 3, generator=g).bfloat16(), "bias": torch.zeros(16).bfloat16()})
         x = torch.randn(4, 16, generator=g)  # fp32 activations on bf16 storage: manual cast in the parent's forward
-        n0 = B.DEFERRED
+        n0, p0 = B.DEFERRED, bo.parent_forwards
         y = lin(x)
-        assert B.DEFERRED == n0 + 1 and y.dtype == torch.float32
+        assert B.DEFERRED == n0 + 1 and bo.parent_forwards == p0 + 1 and y.dtype == torch.float32
         assert_close("manual-cast Linear through the parent's forward", y, torch.nn.functional.linear(x, wl.float(), bl.float()), max_abs=1e-5)
         assert conv(torch.randn(1, 8, 8, 8, generator=g)).dtype == torch.float32
+        assert B.DEFERRED == n0 + 2 and bo.parent_forwards == p0 + 2
         lin.parameters_manual_cast = False
+        assert B._plain(lin)
         lin.forge_online_loras = {}
         assert not B._plain(lin)
     finally:

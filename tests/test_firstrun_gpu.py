@@ -20,7 +20,8 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _gold(name):
-    return torch.load(os.path.join(GOLD, name), weights_only=False)
+    from oracle.golden import load_golden
+    return load_golden(name)
 
 
 def _rand(*shape, dtype=torch.float16, scale=1.0, seed=0):

@@ -7,7 +7,6 @@ import types
 import pytest
 import torch
 
-from oracle import ref_import
 from oracle import sampling as S
 from tests.util import assert_close
 
@@ -119,25 +118,39 @@ def test_plugin_installs_samplers_and_defers_unsupported_cases():
     assert ks.sample_dpmpp_2m(None, x, torch.tensor([1.0, 0.0])) == "ref_dpmpp"
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted")
-def test_plugin_binds_into_the_real_reference_modules():
-    """With the actual reference imported: the names Forge's UNet/VAE call resolve to the B200 functions after
-    install(), and CPU calls (outside the fused path) still produce the reference's own results."""
-    ref_import.load()
-    import backend.attention as ba
-    import backend.nn.unet as bu
+def test_plugin_binds_into_the_real_reference_modules(monkeypatch):
+    """The modules that import attention_function by value in the reference (recorded in tests/golden/plugin_calls.pt):
+    after install() every one of them resolves to the B200 functions, and CPU calls (outside the fused path) still produce
+    the reference's own results."""
     from b200forge import attention as A
     from b200forge import plugin
+    from oracle import ops as O
+    from oracle.golden import load_golden
+    g = load_golden("plugin_calls.pt")
+
+    def attention_pytorch(q, k, v, heads, mask=None, attn_precision=None, skip_reshape=False):
+        return O.attention(q, k, v, heads)
+
+    def attention_pytorch_single_head_spatial(q, k, v):
+        raise AssertionError("not called here")
+
+    for name in ["backend.attention"] + g["attention_importers"] + g["single_head_importers"]:
+        monkeypatch.setitem(sys.modules, name, types.ModuleType(name))
+    for name in ["backend.attention"] + g["attention_importers"]:
+        sys.modules[name].attention_function = attention_pytorch
+    for name in ["backend.attention"] + g["single_head_importers"]:
+        sys.modules[name].attention_function_single_head_spatial = attention_pytorch_single_head_spatial
     plugin.install_attention()
     try:
-        assert bu.attention_function is A.attention_function and ba.attention_function is A.attention_function
-        q = torch.randn(2, 16, 128)
-        out = bu.attention_function(q, q, q, 2)
-        from oracle import ops as O
-        assert_close("deferred attention == reference", out, O.attention(q, q, q, 2), max_abs=1e-5)
+        assert all(sys.modules[n].attention_function is A.attention_function for n in ["backend.attention"] + g["attention_importers"])
+        assert all(sys.modules[n].attention_function_single_head_spatial is A.attention_function_single_head_spatial
+                   for n in ["backend.attention"] + g["single_head_importers"])
+        q = g["deferred_q"]
+        out = sys.modules["backend.nn.unet"].attention_function(q, q, q, 2)
+        assert_close("deferred attention == reference", out, g["deferred_out"], max_abs=1e-5)
     finally:
         plugin.uninstall_attention()
-    assert bu.attention_function.__name__ == "attention_pytorch"
+    assert sys.modules["backend.nn.unet"].attention_function.__name__ == g["attention_function_name"] == "attention_pytorch"
 
 
 def test_operations_class_surface_and_cpu_deferral():
@@ -341,17 +354,22 @@ def test_k_sampler_host_logic_vs_reference_golden(key, monkeypatch):
     assert err <= 2e-5 * max(1.0, scale), (key, err, scale)
 
 
-@pytest.mark.skipif(not ref_import.available(), reason="reference tree not mounted (the dispatch is on the reference's PredictionFlux type)")
 @pytest.mark.parametrize("name", ["sample_euler_ancestral", "sample_dpm_2_ancestral"])
 def test_rectified_flow_ancestral_samplers_vs_reference_golden(name, monkeypatch):
     """For a Flux model the reference's Euler a / DPM2 a switch to their rectified-flow variants
-    (k_diffusion/sampling.py:143-144, 162-186, 251-252, 278-309); the fused versions dispatch the same way."""
+    (k_diffusion/sampling.py:143-144, 162-186, 251-252, 278-309); the fused versions dispatch the same way.  The dispatch is
+    on the predictor's type, backend.modules.k_prediction.PredictionFlux, stood in for here by a class of that name."""
     import os
 
     import torch
 
-    ref_import.load()
-    from backend.modules.k_prediction import PredictionFlux
+    k_prediction = types.ModuleType("backend.modules.k_prediction")
+
+    class PredictionFlux:
+        prediction_type = "const"
+
+    k_prediction.PredictionFlux = PredictionFlux
+    monkeypatch.setitem(sys.modules, "backend.modules.k_prediction", k_prediction)
 
     from b200forge import k_samplers
     from oracle import sampling as OS
