@@ -299,9 +299,14 @@ int b200_tile_resolve(const float* acc, float* out, size_t pixels, int accumulat
  * (255 * x, astype(uint8): truncation); doing it on the device quarters the bytes that leave the GPU.  n % 4 == 0. */
 int b200_images_to_u8(const float* x, unsigned char* out, size_t n, b200_stream_t s);
 
-/* ControlNet residual: h NHWC [N, H, W, C] (dtype) += ctrl NCHW [N, C, H, W] (dtype, or fp32 when ctrl_is_f32)
- * (backend/nn/unet.py:44-52 apply_control on the input / middle / output-skip activations).  C multiple of 8.
- * Added after the round's GPU budget was spent: exercised so far only through the CPU emulation of the engine. */
+/* Control residual, in place: h NHWC [N, H, W, C] (dtype) += ctrl, with ctrl NCHW [ctrl_batch, C, H, W] or, when ctrl_nhwc,
+ * NHWC [ctrl_batch, H, W, C] (16-byte aligned); dtype, or fp32 when ctrl_is_f32.  ctrl_batch is N or 1: a batch-1 residual
+ * is added to every image, as torch's broadcasting `h += ctrl` does (backend/nn/unet.py:44-52 apply_control on the
+ * input / middle / output-skip activations, T2I-Adapter residuals of one hint image; backend/nn/cnets/cldm.py:259-262
+ * `h += guided_hint`).  C multiple of 8. */
+int b200_add_control(void* h, const void* ctrl, int N, int C, int H, int W, int ctrl_batch, int ctrl_nhwc, int ctrl_is_f32,
+                     int dtype, b200_stream_t s);
+/* b200_add_control with an NCHW residual of batch N. */
 int b200_add_nchw(void* h, const void* ctrl, int N, int C, int H, int W, int ctrl_is_f32, int dtype, b200_stream_t s);
 
 /* VAE encode entry: pixels NHWC fp32 [pixels, 3] in [0, 1] -> [pixels, 8] in dtype, channels 0-2 = 2x - 1, 3-7 = 0

@@ -593,11 +593,13 @@ __global__ void vae_posterior_kernel(const void* __restrict__ mom, const float* 
   }
 }
 
-// ControlNet residual (backend/nn/unet.py:44-52 apply_control, `h += ctrl`): h NHWC [N, H, W, C] (dtype) accumulates a
-// control tensor that arrives in the reference's NCHW layout (dtype or fp32).  One thread per 8 channels of one pixel.
+// Control residual, `h += ctrl` (backend/nn/unet.py:44-52 apply_control; cldm.py:259-262 `h += guided_hint`): h NHWC
+// [N, H, W, C] (dtype) accumulates a control tensor in the reference's NCHW layout or channels-last (ctrl_nhwc), dtype or
+// fp32, whose batch is N or 1 (ctrl_batch1: one image broadcast over the batch, as torch's in-place add does).  One thread
+// per 8 channels of one pixel.
 template <bool BF16>
-__global__ void add_nchw_kernel(void* __restrict__ h, const void* __restrict__ ctrl, int N, int C, int H, int W,
-                                int ctrl_is_f32) {
+__global__ void add_control_kernel(void* __restrict__ h, const void* __restrict__ ctrl, int N, int C, int H, int W,
+                                   int ctrl_batch1, int ctrl_nhwc, int ctrl_is_f32) {
   const int CV = C >> 3;
   const size_t HW = (size_t)H * W;
   const size_t total = (size_t)N * HW * CV;
@@ -605,13 +607,27 @@ __global__ void add_nchw_kernel(void* __restrict__ h, const void* __restrict__ c
     const int cv = (int)(i % CV);
     const size_t t = i / CV;
     const size_t hw = t % HW;
-    const size_t n = t / HW;
+    const size_t n = ctrl_batch1 ? 0 : t / HW;  // batch index into ctrl
     float v[8];
     load8<BF16>(h, i * 8, v);
+    if (ctrl_nhwc) {
+      const size_t src = (n * HW + hw) * C + (size_t)cv * 8;
+      float u[8];
+      if (ctrl_is_f32) {
+        const float4 a = *reinterpret_cast<const float4*>(reinterpret_cast<const float*>(ctrl) + src);
+        const float4 b = *reinterpret_cast<const float4*>(reinterpret_cast<const float*>(ctrl) + src + 4);
+        u[0] = a.x; u[1] = a.y; u[2] = a.z; u[3] = a.w; u[4] = b.x; u[5] = b.y; u[6] = b.z; u[7] = b.w;
+      } else {
+        load8<BF16>(ctrl, src, u);
+      }
 #pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const size_t src = (n * C + (size_t)(cv * 8 + j)) * HW + hw;
-      v[j] += ctrl_is_f32 ? reinterpret_cast<const float*>(ctrl)[src] : ld1<BF16>(ctrl, src);
+      for (int j = 0; j < 8; ++j) v[j] += u[j];
+    } else {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const size_t src = (n * C + (size_t)(cv * 8 + j)) * HW + hw;
+        v[j] += ctrl_is_f32 ? reinterpret_cast<const float*>(ctrl)[src] : ld1<BF16>(ctrl, src);
+      }
     }
     store8<BF16>(h, i * 8, v);
   }
@@ -879,11 +895,20 @@ extern "C" int b200_vae_posterior(const void* moments, const float* noise, float
   return B200_OK;
 }
 
+extern "C" int b200_add_control(void* h, const void* ctrl, int N, int C, int H, int W, int ctrl_batch, int ctrl_nhwc,
+                                int ctrl_is_f32, int dtype, b200_stream_t s) {
+  B200_CHECK_ARG(h && ctrl && N > 0 && C > 0 && H > 0 && W > 0 && C % 8 == 0,
+                 "add_control: bad arguments (C must be a multiple of 8)");
+  B200_CHECK_ARG(ctrl_batch == N || ctrl_batch == 1, "add_control: residual batch %d must be 1 or %d", ctrl_batch, N);
+  B200_CHECK_ARG(!ctrl_nhwc || (reinterpret_cast<uintptr_t>(ctrl) & 15) == 0, "add_control: NHWC residual must be 16-byte aligned");
+  const size_t total = (size_t)N * H * W * (C / 8);
+  DISPATCH_DTYPE(dtype, add_control_kernel<BF><<<grid_for(total, 256), 256, 0, (cudaStream_t)s>>>(
+                            h, ctrl, N, C, H, W, ctrl_batch == 1 && N > 1 ? 1 : 0, ctrl_nhwc ? 1 : 0, ctrl_is_f32));
+  B200_CHECK_LAUNCH("add_control");
+  return B200_OK;
+}
+
 extern "C" int b200_add_nchw(void* h, const void* ctrl, int N, int C, int H, int W, int ctrl_is_f32, int dtype,
                              b200_stream_t s) {
-  B200_CHECK_ARG(h && ctrl && N > 0 && C > 0 && H > 0 && W > 0 && C % 8 == 0, "add_nchw: bad arguments (C must be a multiple of 8)");
-  const size_t total = (size_t)N * H * W * (C / 8);
-  DISPATCH_DTYPE(dtype, add_nchw_kernel<BF><<<grid_for(total, 256), 256, 0, (cudaStream_t)s>>>(h, ctrl, N, C, H, W, ctrl_is_f32));
-  B200_CHECK_LAUNCH("add_nchw");
-  return B200_OK;
+  return b200_add_control(h, ctrl, N, C, H, W, N, 0, ctrl_is_f32, dtype, s);
 }

@@ -120,6 +120,7 @@ SIGNATURES = {
     "b200_sampler_update": (_i, [_vp, _vp, _vp, _vp, C.POINTER(StepDesc), _vp]),
     "b200_eps_to_denoised": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "b200_add_nchw": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "b200_add_control": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "b200_vae_preprocess": (_i, [_vp, _vp, _sz, _i, _vp]),
     "b200_vae_posterior": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _vp]),
     "b200_adaln": (_i, [_vp, _vp, _i, _i, _f, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),

@@ -761,15 +761,23 @@ def images_to_u8(img: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch
     return out
 
 
-def add_nchw_(h: torch.Tensor, ctrl: torch.Tensor) -> torch.Tensor:
-    """h NHWC [N,H,W,C] += ctrl NCHW [N,C,H,W] (same dtype as h, or fp32), in place."""
+def add_control_(h: torch.Tensor, ctrl: torch.Tensor, *, nhwc: bool = False) -> torch.Tensor:
+    """h NHWC [N,H,W,C] += ctrl, in place: ctrl NCHW [N|1,C,H,W] or (nhwc) NHWC [N|1,H,W,C], h.dtype or fp32; a batch-1
+    residual is added to every image."""
     assert h.dim() == 4 and h.is_contiguous() and ctrl.is_contiguous()
     n, hh, ww, c = h.shape
-    assert tuple(ctrl.shape) == (n, c, hh, ww) and ctrl.dtype in (h.dtype, torch.float32)
-    _l.check(_l.load().b200_add_nchw(h.data_ptr(), ctrl.data_ptr(), n, c, hh, ww, 1 if ctrl.dtype == torch.float32 else 0,
-                                     _dt(h), _stream()))
+    nc = ctrl.shape[0]
+    assert nc in (n, 1) and tuple(ctrl.shape[1:]) == ((hh, ww, c) if nhwc else (c, hh, ww)), (tuple(h.shape), tuple(ctrl.shape))
+    assert ctrl.dtype in (h.dtype, torch.float32)
+    _l.check(_l.load().b200_add_control(h.data_ptr(), ctrl.data_ptr(), n, c, hh, ww, nc, 1 if nhwc else 0,
+                                        1 if ctrl.dtype == torch.float32 else 0, _dt(h), _stream()))
     _count()
     return h
+
+
+def add_nchw_(h: torch.Tensor, ctrl: torch.Tensor) -> torch.Tensor:
+    """h NHWC [N,H,W,C] += ctrl NCHW [N|1,C,H,W] (same dtype as h, or fp32), in place."""
+    return add_control_(h, ctrl)
 
 
 def vae_preprocess(pixels: torch.Tensor, dtype: torch.dtype, out: Optional[torch.Tensor] = None) -> torch.Tensor:

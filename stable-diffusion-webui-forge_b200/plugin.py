@@ -49,8 +49,9 @@ def fast_path_ok(c: dict) -> bool:
 
 def _control_ok(control) -> bool:
     """ControlNet / T2I-Adapter residuals the fused UNet can add itself (UNetEngine.forward_cols(control=...)): a dict of
-    lists of CUDA tensors / None under the reference's three names (backend/nn/unet.py:44-52).  B200_CONTROL=0 sends such
-    calls to Forge's own forward instead."""
+    lists of CUDA tensors / None under the reference's three names (backend/nn/unet.py:44-52); their shapes (the
+    activation's, with its batch or batch 1) are checked against the latent by UNetEngine.control_fits.  B200_CONTROL=0
+    sends such calls to Forge's own forward instead."""
     import os
     if os.environ.get("B200_CONTROL") == "0" or not isinstance(control, dict):
         return False
@@ -224,6 +225,7 @@ class UNetWrapper:
         if (not fast_path_ok(c) or not _on_device(x) or x.dtype != torch.float32 or ptype not in ("epsilon", "v_prediction")
                 or (self.engine.has_label and c.get("y") is None) or x.dim() != 4
                 or not self.engine.supports_latent(x.shape[2], x.shape[3])
+                or (c.get("control") is not None and not self.engine.control_fits(c["control"], x.shape[0], x.shape[2], x.shape[3]))
                 or (self.weights is not None and not self.weights.servable())):
             self.calls_reference += 1
             return apply_model_fn(x, sigma, **c)
@@ -317,6 +319,87 @@ def install_flux_wrapper(unet_patcher, engine=None) -> FluxWrapper:
                             device=unet_patcher.load_device)
     w = FluxWrapper(engine, kmodel.predictor, kmodel)
     unet_patcher.set_model_unet_function_wrapper(w)
+    return w
+
+
+# ------------------------------------------------------------------------------------------------- P6 ControlNet model
+class ControlNetWrapper:
+    """`transformer_options['controlnet_model_function_wrapper']` (set by UnetPatcher.set_controlnet_model_function_wrapper,
+    backend/patcher/unet.py:169-170; copied onto every ControlNet of the chain, sampling_function.py:261-268):
+    ControlNet.get_control calls wrapper(x=, hint=, timesteps=, context=, y=, model=, inner_model=) instead of
+    `control_model(...)` (backend/patcher/controlnet.py:329-339) and hands the result to control_merge, which keeps strength,
+    per-block / per-sigma weighting, masks, global average pooling and the merging of several ControlNets.
+
+    One ControlNetEngine per control model (built on its first fast call from `inner_model.state_dict()`).  A call is
+    handed back exactly as get_control's own no-wrapper branch would run it when it is a T2I-Adapter call
+    (`inner_t2i_model`, controlnet.py:524-531), a Control-LoRA, on a tensor that is not on CUDA, in a dtype other than
+    fp16 / bf16, at a latent size the engine does not tile, with a hint that is not 8x the latent, for a model whose
+    engine could not be built (B200_STRICT=1: that raises instead), or when B200_CONTROLNET=0.  What is decided per
+    model (Control-LoRA or not, engine built or not) is decided once, on its first call."""
+
+    def __init__(self):
+        import weakref
+        self.engines = weakref.WeakKeyDictionary()  # inner_model -> ControlNetEngine
+        self.unserved = weakref.WeakKeyDictionary()  # inner_model -> why its calls go back to Forge (Control-LoRA, build error)
+        self.calls_fast = 0
+        self.calls_reference = 0
+
+    @staticmethod
+    def _is_control_lora(model, inner_model) -> bool:
+        if type(model).__name__ == "ControlLora":
+            return True
+        mods = getattr(inner_model, "modules", None)
+        return mods is not None and any(hasattr(m, "up") and hasattr(m, "down") for m in inner_model.modules())
+
+    def _engine(self, model, inner_model, x):
+        """The engine of `inner_model` in x's dtype on x's device, or None when its calls go back to Forge."""
+        import os
+        from .controlnet_engine import ControlNetEngine, controlnet_config
+        if inner_model in self.unserved:
+            return None
+        eng = self.engines.get(inner_model)
+        if eng is None or eng.dtype != x.dtype or eng.device != x.device:
+            if self._is_control_lora(model, inner_model):
+                self.unserved[inner_model] = "Control-LoRA"
+                return None
+            try:
+                eng = ControlNetEngine(controlnet_config(inner_model), inner_model.state_dict(), dtype=x.dtype, device=x.device)
+            except Exception as e:
+                if os.environ.get("B200_STRICT") == "1":
+                    raise
+                self.unserved[inner_model] = f"engine not built: {type(e).__name__}: {e}"
+                return None
+            self.engines[inner_model] = eng
+        return eng
+
+    def __call__(self, x=None, hint=None, timesteps=None, context=None, y=None, model=None, inner_model=None, **kw):
+        import os
+        if "inner_t2i_model" in kw:  # T2I-Adapter: runs once per job on the hint alone (controlnet.py:531)
+            self.calls_reference += 1
+            dev = getattr(model, "device", None)
+            return inner_model(hint if dev is None else hint.to(dev))
+        tensors = [x, timesteps, context] + ([] if y is None else [y])
+        eng = None
+        if (os.environ.get("B200_CONTROLNET") != "0" and type(model).__name__ != "ControlLora"
+                and all(torch.is_tensor(t) and _on_device(t) for t in tensors) and torch.is_tensor(hint)
+                and x.dim() == 4 and x.dtype in (torch.float16, torch.bfloat16)):
+            eng = self._engine(model, inner_model, x)
+            if eng is not None and not (eng.supports_latent(x.shape[2], x.shape[3]) and eng.supports_hint(hint, x.shape[0], x.shape[2], x.shape[3])
+                    and (y is not None or not eng.has_label)):
+                eng = None
+        if eng is None:
+            self.calls_reference += 1
+            dev = getattr(model, "device", None)
+            return inner_model(x=x, hint=hint if dev is None else hint.to(dev), timesteps=timesteps, context=context, y=y)
+        self.calls_fast += 1
+        return eng.forward(x, hint, timesteps, context, y)
+
+
+def install_controlnet_wrapper(unet_patcher) -> ControlNetWrapper:
+    """Serve every ControlNet model of the jobs this UnetPatcher runs from the fused engine (P6).  The wrapper lives in
+    the patcher's transformer_options, so clones made per generation (LoRA, ControlNet units) inherit it."""
+    w = ControlNetWrapper()
+    unet_patcher.set_controlnet_model_function_wrapper(w)
     return w
 
 

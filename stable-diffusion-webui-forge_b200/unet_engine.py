@@ -34,16 +34,16 @@ from .ops import EPI_GEGLU, EPI_NONE, EPI_SILU
 SD = Dict[str, torch.Tensor]
 
 
-def unet_structure(cfg: dict):
-    """Block list of the LDM UNet for a config (mirrors the constructor order of backend/nn/unet.py:481-693):
-    ("conv"|"res"|"attn"|"down"|"up", prefix, ...)."""
+def encoder_structure(cfg: dict):
+    """Input blocks and middle block of the LDM UNet encoder, shared by the UNet and by cldm.ControlNet, whose constructors
+    build them in the same order (backend/nn/unet.py:481-620, backend/nn/cnets/cldm.py:131-234):
+    (input, middle, chans, ch) with chans the channel count after every input block and ch the middle block's."""
     mc = cfg["model_channels"]
     nrb = cfg["num_res_blocks"]
     cm = list(cfg["channel_mult"])
     if isinstance(nrb, int):
         nrb = len(cm) * [nrb]
     td = list(cfg["transformer_depth"])
-    tdo = list(cfg["transformer_depth_output"])
     nh, nhc = cfg["num_heads"], cfg["num_head_channels"]
 
     def heads_of(ch):
@@ -73,6 +73,24 @@ def unet_structure(cfg: dict):
     if cfg["transformer_depth_middle"] >= 0:
         mid += [("attn", "middle_block.1", ch, h, dh, cfg["transformer_depth_middle"]),
                 ("res", "middle_block.2", ch, ch)]
+    return inp, mid, chans, ch
+
+
+def unet_structure(cfg: dict):
+    """Block list of the LDM UNet for a config (mirrors the constructor order of backend/nn/unet.py:481-693):
+    ("conv"|"res"|"attn"|"down"|"up", prefix, ...)."""
+    mc = cfg["model_channels"]
+    nrb = cfg["num_res_blocks"]
+    cm = list(cfg["channel_mult"])
+    if isinstance(nrb, int):
+        nrb = len(cm) * [nrb]
+    tdo = list(cfg["transformer_depth_output"])
+    nh, nhc = cfg["num_heads"], cfg["num_head_channels"]
+
+    def heads_of(ch):
+        return (nh, ch // nh) if nhc == -1 else (ch // nhc, nhc)
+
+    inp, mid, chans, ch = encoder_structure(cfg)
     out = []
     i = 0
     for level, mult in list(enumerate(cm))[::-1]:
@@ -100,7 +118,7 @@ class UNetEngine:
         self.cfg = dict(cfg)
         self.dtype = dtype
         self.device = torch.device(device)
-        self.st = unet_structure(cfg)
+        self.st = self._structure(cfg)
         self.mc = cfg["model_channels"]
         self.ted = self.mc * 4
         self.has_label = cfg.get("num_classes") is not None
@@ -109,6 +127,10 @@ class UNetEngine:
         if self.device.type == "cuda":
             ops.gn_workspace(self.device)  # created (zeroed) here so that it never happens inside a graph capture
         self._pack(state_dict)
+
+    @staticmethod
+    def _structure(cfg: dict) -> dict:
+        return unet_structure(cfg)
 
     # ------------------------------------------------------------------------------------------ packing
     def repack(self, state_dict: SD) -> None:
@@ -123,11 +145,31 @@ class UNetEngine:
     def _pack(self, sd: SD) -> None:
         w = self.w
         g = lambda k: self._t(sd[k])  # noqa: E731
+        self._pack_embeddings(g)
+        self._pack_blocks(g, self.st["input"] + [self.st["middle"]] + self.st["output"])
+        w["out.0.g"], w["out.0.b"] = g("out.0.weight"), g("out.0.bias")
+        ow = ops.pack_conv3x3(g("out.2.weight"))  # [4, 9*mc] -> pad to 8 output channels
+        co = ow.shape[0]
+        self.out_channels = co
+        owp = torch.zeros((8, ow.shape[1]), dtype=self.dtype, device=self.device)
+        owp[:co] = ow
+        obp = torch.zeros((8,), dtype=self.dtype, device=self.device)
+        obp[:co] = g("out.2.bias")
+        w["out.2.w"], w["out.2.b"] = owp, obp
+
+    def _pack_embeddings(self, g) -> None:
+        """time_embed and label_emb; `g(name)` returns the state-dict tensor on the device in the compute dtype."""
+        w = self.w
         for p in ("time_embed.0", "time_embed.2"):
             w[p + ".w"], w[p + ".b"] = g(p + ".weight"), g(p + ".bias")
         if self.has_label:
             for p in ("label_emb.0.0", "label_emb.0.2"):
                 w[p + ".w"], w[p + ".b"] = g(p + ".weight"), g(p + ".bias")
+
+    def _pack_blocks(self, g, blocks) -> None:
+        """Every layer of `blocks` (lists of structure tuples), plus all their ResBlock time-embedding projections stacked
+        into one matrix, in block order."""
+        w = self.w
         emb_w, emb_b = [], []
         self.emb_off: Dict[str, tuple] = {}
         off = 0
@@ -213,20 +255,11 @@ class UNetEngine:
                     w[p + ".w"] = ops.pack_conv3x3(g(p + ".conv.weight"))
                 w[p + ".b"] = g(p + ".conv.bias")
 
-        for blk in self.st["input"] + [self.st["middle"]] + self.st["output"]:
+        for blk in blocks:
             for layer in blk:
                 pack_layer(layer)
         w["emb_all.w"] = torch.cat(emb_w, 0).contiguous()
         w["emb_all.b"] = torch.cat(emb_b, 0).contiguous()
-        w["out.0.g"], w["out.0.b"] = g("out.0.weight"), g("out.0.bias")
-        ow = ops.pack_conv3x3(g("out.2.weight"))  # [4, 9*mc] -> pad to 8 output channels
-        co = ow.shape[0]
-        self.out_channels = co
-        owp = torch.zeros((8, ow.shape[1]), dtype=self.dtype, device=self.device)
-        owp[:co] = ow
-        obp = torch.zeros((8,), dtype=self.dtype, device=self.device)
-        obp[:co] = g("out.2.bias")
-        w["out.2.w"], w["out.2.b"] = owp, obp
 
     # ------------------------------------------------------------------------------------------ blocks
     def _res(self, p: str, layer, x1: torch.Tensor, x2: Optional[torch.Tensor], temb_all: torch.Tensor) -> torch.Tensor:
@@ -360,10 +393,39 @@ class UNetEngine:
         # every ResBlock applies Linear(SiLU(emb)) (unet.py:412-415): one stacked GEMM for all of them
         return ops.gemm(ops.silu(emb), w["emb_all.w"], w["emb_all.b"])
 
+    def control_fits(self, control: dict, n: int, hh: int, ww: int) -> bool:
+        """Whether every residual that forward_cols would add for an [n, *, hh, ww] latent is an NCHW tensor of its
+        activation's shape, or of batch 1 (added to every image, as the reference's broadcasting `h += ctrl` does), in the
+        compute dtype or fp32.  The reference prints "could not be applied" and skips any other residual (apply_control,
+        backend/nn/unet.py:44-52): callers hand such calls to Forge's own forward, which does exactly that."""
+        shapes = []  # (channels, height, width) after each input block
+        c, h, w = self.cfg["in_channels"], hh, ww
+        for layers in self.st["input"]:
+            for layer in layers:
+                if layer[0] in ("conv", "res"):
+                    c = layer[3]
+                elif layer[0] == "down":
+                    h, w = (h + 1) // 2, (w + 1) // 2
+            shapes.append((c, h, w))
+
+        def fits(name, wanted):  # wanted: activation shapes in the order the residuals are popped
+            lst = list(control.get(name) or [])
+            for shp in wanted:
+                if not lst:
+                    return True
+                t = lst.pop()
+                if t is not None and not (torch.is_tensor(t) and t.dim() == 4 and t.shape[0] in (n, 1)
+                                          and tuple(t.shape[1:]) == shp and t.dtype in (self.dtype, torch.float32)):
+                    return False
+            return True
+
+        return (fits("input", shapes) and fits("middle", [(c, h, w)])
+                and fits("output", shapes[::-1][:len(self.st["output"])]))
+
     @staticmethod
     def _apply_control(h: torch.Tensor, control: Optional[dict], name: str) -> torch.Tensor:
         """apply_control (backend/nn/unet.py:44-52): pop the LAST tensor of control[name] and add it in place; the
-        residual arrives NCHW, `h` is channels-last."""
+        residual arrives NCHW with h's batch or batch 1 (see control_fits), `h` is channels-last."""
         if control is not None and name in control and len(control[name]) > 0:
             ctrl = control[name].pop()
             if ctrl is not None:
